@@ -34,6 +34,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True          # the tree may be read-only; nothing is cached in it
 PROFILE_JSON = "r02_kernels.json"       # the committed ncu --set full summary the roofline's `traffic` comes from
 PROFILE_FALLBACK = "r01k_kernels.json"
 sys.path.insert(0, ROOT)
@@ -43,6 +44,7 @@ W = H = 8192
 NC, BD, LEVELS = 3, 12, 5
 WORKLOAD = ("8192x8192x3 12-bit, reversible 5/3 + RCT, 5 levels, 64x64 code-blocks, RPCL; a step = a batch of "
             "independent frames, each encoded then decoded")
+DUMP_SAMPLES = 1 << 22                  # --dump-outputs: codestream bytes sampled; half as many samples per component
 CONFIG = {"workload": WORKLOAD, "l2_policy": "inputs larger than L2 (402 MB frame, 805 MB coefficients)"}
 
 
@@ -484,6 +486,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last device-resident step of the headline returned as DIR/*.npy: "
+                         "the codestream's length, its first 64 KiB and a fixed sample of its bytes, and a fixed sample of the "
+                         "decoded samples of every component (positions drawn with numpy's default_rng(0); about 40 MB)")
     a = ap.parse_args()
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -621,7 +627,31 @@ def main():
         pass
     peak = float(peaks.get("hbm_gbs", 6650.0)); peak_src = "measured (MEASURED_PEAKS.json)" if peaks else "fallback 6650 GB/s"
 
-    def measure(wl, steps, warmup, lossless, e2e=True):
+    class DeviceArray:
+        """a view of device memory the library owns, for torch.as_tensor"""
+        def __init__(self, ptr, n, typestr):
+            self.__cuda_array_interface__ = {"data": (int(ptr), False), "shape": (n,), "typestr": typestr, "version": 2}
+
+    def resident_outputs(w):
+        """what one device-resident step hands its caller: the codestream in device memory and the decoded planes in the
+        decoder's image buffer, sampled at seeded positions so that two builds compare output for output"""
+        wl, n = w.wl, int(w.n.value)
+        rng = np.random.default_rng(0)
+        pos = torch.from_numpy(np.sort(rng.integers(0, n, DUMP_SAMPLES))).cuda()
+        out = {"codestream_length": np.array([n], np.float64),
+               "codestream_head": w.cs_dev[:min(n, 1 << 16)].float().cpu().numpy(),
+               "codestream_sample": w.cs_dev[pos].float().cpu().numpy()}
+        h, wd = wl.frame[0].shape
+        pix = torch.from_numpy(np.sort(rng.integers(0, h * wd, DUMP_SAMPLES // 2))).cuda()
+        typestr = "|u1" if wl.st == ob.U8 else "<i2"
+        for c in range(wl.nc):
+            plane = torch.as_tensor(DeviceArray(L.ojb_dec_device_plane(w.dec, c), h * wd, typestr), device="cuda")
+            v = plane[pix].to(torch.int32)
+            out["decoded_c%d" % c] = (v & 0xFFFF if typestr == "<i2" else v).float().cpu().numpy()
+        torch.cuda.synchronize()
+        return out
+
+    def measure(wl, steps, warmup, lossless, e2e=True, dump=False):
         """correctness of what is timed, then: serial pass (per-stage CUDA-event times), all workers in flight
         resident (`value`), all workers in flight through host buffers (`e2e`)"""
         ws = wl.workers
@@ -647,7 +677,8 @@ def main():
         dt_serial = timed(ws[:1], "resident", steps)
         L.ojb_enc_timings(ws[0].enc, te); L.ojb_dec_timings(ws[0].dec, td)
         dt_res = timed(ws, "resident", steps)
-        r = {"dt_serial": dt_serial, "dt_res": dt_res, "dt_e2e": None, "te": list(te), "td": list(td), "te2": None, "td2": None,
+        outputs = resident_outputs(ws[0]) if dump else None
+        r = {"outputs": outputs, "dt_serial": dt_serial, "dt_res": dt_res, "dt_e2e": None, "te": list(te), "td": list(td), "te2": None, "td2": None,
              "cs_len": int(ws[0].cs_len), "mirror_bytes": int(L.ojb_dec_mirror_bytes(ws[0].dec))}
         if e2e:
             for _ in range(max(1, min(warmup, 2))):
@@ -691,7 +722,11 @@ def main():
     frame = make_frame(W, H, 1234 + rank)
     head = Workload(p, frame, NW)
     sampler = ClockSampler(local); sampler.start()
-    r = measure(head, a.steps, a.warmup, True)
+    r = measure(head, a.steps, a.warmup, True, dump=bool(a.dump_outputs) and rank == 0)
+    if r["outputs"]:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, arr in r["outputs"].items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), arr)
     sampler.stop_flag = True; sampler.join(timeout=2)
     cs_len = r["cs_len"]
     enc, dec = head.workers[0].enc, head.workers[0].dec

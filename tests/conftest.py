@@ -27,9 +27,10 @@ def emu_lib():
     return emu.emu_lib()
 
 
-@pytest.fixture(scope="session")
-def ref():
+@pytest.fixture
+def ref(request):
+    """the reference's answers: its build in oracle/_ref when present, else the stored ones (tests/refgolden.py),
+    replayed through the library the test checks (the product library in the GPU tier, the emulator build otherwise)"""
     import refharness
-    if not refharness.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
-    return refharness
+    lib = None if "gpu_lib" in request.fixturenames else request.getfixturevalue("emu_lib")
+    return refharness.active(lib)

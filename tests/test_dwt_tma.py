@@ -17,6 +17,7 @@ lib = None
 if %(emu)d:
     import emu
     lib = emu.emu_lib(build=False)
+R = R.active(lib)
 cases = [(1024, 200, 3, 12, dict(num_decomps=4, reversible=True, color_transform=True), ob.U16),
          (1000, 130, 1, 10, dict(num_decomps=3, reversible=True), ob.U16),
          (777, 96, 3, 16, dict(num_decomps=2, reversible=True, color_transform=True, offset=(3, 1)), ob.U16),

@@ -48,13 +48,14 @@ def _worker(rank, world, port, q, which, gpu=False):
         else:
             import emu
             L = emu.emu_lib(build=False)
+        ref = refharness.active(L)
         ok, notes = True, []
 
         def one_encoder(p, fr):
             # the reference's codestream; it has no writer for DFS segments (this library's extension, checked against
             # the reference's DECODER in test_part2_structures.py): there the single-process encoder is the yardstick
             if p.dfs_num_levels == 0:
-                return refharness.encode(p, fr)
+                return ref.encode(p, fr)
             enc = ob.Encoder(p, ob.I32, lib=L)
             try:
                 return enc.encode(fr)
@@ -93,7 +94,7 @@ def _worker(rank, world, port, q, which, gpu=False):
                     ok = ok and cs is None
                 planes = sh.decode(want, sample_type=ob.I32, writer=writer)
                 if rank == writer:
-                    ref_planes, _ = refharness.decode(want)
+                    ref_planes, _ = ref.decode(want)
                     tol = 0 if p.reversible else 1
                     err = max(int(np.abs(a.astype(np.int64) - b).max()) for a, b in zip(planes, ref_planes))
                     if err > tol:
@@ -114,7 +115,7 @@ def _worker(rank, world, port, q, which, gpu=False):
             dist.broadcast_object_list(lens, src=writer)
             sh.decode_resident(addr, lens[0], ob.I32, writer)
             if rank == writer and not gpu:       # (device memory on a GPU: the host-buffer forms above already compared samples)
-                ref_planes, _ = refharness.decode(want if p.reversible else ctypes.string_at(addr, n))
+                ref_planes, _ = ref.decode(want if p.reversible else ctypes.string_at(addr, n))
                 for c, rp in enumerate(ref_planes):
                     got = np.frombuffer(ctypes.string_at(sh.device_plane(c), rp.size * 4), np.int32).reshape(rp.shape)
                     good = np.abs(got.astype(np.int64) - rp).max() <= (0 if p.reversible else 1)
